@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """bench.py — messages/sec through the hot path (parse -> link-extract -> filter/dedup -> JSONL).
 
-Contract (see the task statement):
-    python bench.py [--config {2,3,4,5}] --gpus N --steps K --warmup W [--impl reference]
+Usage:
+    python bench.py [--config {2,3,4,5}] --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 --config selects the BASELINE.json workload (default 2 = configs[1], the configuration the metric is quoted on):
   2  10 M synthetic Telegram mixed text/photo/video-metadata messages per GPU, parse + link-extract + dedup + JSONL
@@ -20,6 +20,8 @@ sharding, no data-path collective) and strong scaling for config 5; the ranks me
     live on the launching stream, against MEASURED_PEAKS.json; plus the whole-step figure (SURVEY.md §8d bytes).
   * cpu_baseline / --impl reference: the CPU oracle (C restatement of the reference's Go path — the reference itself
     cannot be built here, there is no Go toolchain) on the box's host cores, same run flags, same corpus.
+  * --dump-outputs DIR: what the last timed resident step handed its caller, as .npy files (OutputDump): per run the
+    result counts and seeded 4 KB windows of the JSONL, then a seeded sample of the dedup set's keys.
 One JSON line on stdout (rank 0).
 """
 from __future__ import annotations
@@ -43,6 +45,13 @@ GEN_BUDGET_S = float(os.environ.get("TGI_BENCH_GEN_BUDGET_S", 300))  # host time
 ORC_RUN_SLICES, ORC_RUN_PIN = 0x10000, 0x20000
 
 J, L, F, S = 0x01, 0x02, 0x04, 0x10  # TGI_RUN_JSONL / LINKS / FRONTIER / SKIP_SELF
+
+# --dump-outputs: the JSONL and the dedup set of a step are gigabytes, so a fixed, seeded sample of them is written
+# (byte values as float32: at most 43 MB whatever the number of resident runs, small enough to keep beside each build)
+DUMP_SEED = 0x5EED0D0
+DUMP_WINDOW = 4096               # JSONL bytes per sampled window
+DUMP_JSONL_BYTES = 6 << 20       # JSONL bytes sampled over the step, split evenly over its resident runs
+DUMP_FRONTIER_ROWS = 1 << 17     # dedup-set keys sampled (32 bytes each)
 
 
 def configs():
@@ -178,6 +187,58 @@ def host_cpus() -> tuple[int, str]:
     return n, why
 
 
+def stratified(n_items: int, k: int, rng) -> "np.ndarray":
+    """k sorted indices in [0, n_items): one uniformly drawn index in each of k equal strata (all of them if k >= n_items)"""
+    import numpy as np
+    if k >= n_items:
+        return np.arange(n_items, dtype=np.int64)
+    return np.minimum((np.arange(k) + rng.random(k)) * (n_items / k), n_items - 1).astype(np.int64)
+
+
+class OutputDump:
+    """What the timed path hands its caller in one step, for --dump-outputs.  Per resident run: the result counts and
+    seeded windows of the JSONL the run left on the device; after the step: a seeded sample of the dedup set's keys
+    (the merged global set when the ranks merge).  Same arguments -> same corpus -> same windows and rows, so two
+    builds can be compared file by file."""
+
+    def __init__(self, eng, n_runs: int):
+        import numpy as np
+        self.eng, self.np = eng, np
+        self.windows_per_run = max(1, DUMP_JSONL_BYTES // DUMP_WINDOW // n_runs)
+        self.counts, self.at, self.windows = [], [], []
+
+    def run(self, slot, r):
+        """sample run r right after it returned, before the next run reuses its slot"""
+        np = self.np
+        k = len(self.counts)
+        self.counts.append([r.n, r.jsonl_len, r.n_links, r.n_new, r.frontier_size])
+        if not r.jsonl_len:
+            return
+        w = min(DUMP_WINDOW, r.jsonl_len)
+        rng = np.random.default_rng([DUMP_SEED, k])
+        for off in stratified(r.jsonl_len - w + 1, self.windows_per_run, rng):
+            row = np.full(DUMP_WINDOW, -1.0, np.float32)  # -1: past the end of a JSONL shorter than one window
+            row[:w] = np.frombuffer(self.eng.read_jsonl(slot, int(off), w), np.uint8)
+            self.windows.append(row)
+            self.at.append([k, off])
+
+    def write(self, out_dir: str, keys):
+        """keys: the (n, 32) uint8 dedup set after the step"""
+        np = self.np
+        rows = stratified(len(keys), DUMP_FRONTIER_ROWS, np.random.default_rng([DUMP_SEED, 1 << 20]))
+        arrays = {
+            "run_counts": np.array(self.counts, np.float64).reshape(-1, 5),  # n, jsonl_len, n_links, n_new, frontier_size
+            "jsonl_window_at": np.array(self.at, np.float64).reshape(-1, 2),  # run, byte offset of the window
+            "jsonl_windows": np.array(self.windows, np.float32).reshape(-1, DUMP_WINDOW),
+            "frontier_rows": rows.astype(np.float64),
+            "frontier_keys": keys[rows].astype(np.float32),
+        }
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+        return sum(a.nbytes for a in arrays.values())
+
+
 def make_corpus(cfg, n, first, threads):
     from distributed_crawler_b200.corpus import Corpus, YtCorpus
     if cfg["kind"] == "yt":
@@ -267,15 +328,26 @@ def run_reference(args, cfg, rank):
 
 
 def main():
+    def positive(s):
+        v = int(s)
+        if v < 1:
+            raise argparse.ArgumentTypeError("must be at least 1")
+        return v
+
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=positive, default=5, help="timed steps of the resident leg and of the host-buffer leg")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--config", type=int, default=2, choices=[2, 3, 4, 5])
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer leg (profiling runs)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of what the last resident step computed as "
+                         "DIR/<name>.npy; the corpus is then never cut to the generator's time budget")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -320,7 +392,9 @@ def main():
     want_json = bool(RUN & J)
     n = cfg["n"] // world if cfg["scaling"] == "strong" else cfg["n"]   # records per GPU
     n_asked = n
-    if n > 4_000_000:  # the corpus is generated on the host: keep that inside a time budget, whatever CPUs this box grants
+    # the corpus is generated on the host: keep that inside a time budget, whatever CPUs this box grants; a dump must
+    # see the same corpus on every run, so it takes the configured size
+    if n > 4_000_000 and not args.dump_outputs:
         t_probe = time.perf_counter()
         make_corpus(cfg, 1_000_000, rank * n, gen_threads).close()
         rate = 1_000_000 / (time.perf_counter() - t_probe)
@@ -367,7 +441,7 @@ def main():
             self.launches = 0
             self.ms = {"kernel": 0.0, "parse": 0.0, "emit": 0.0, "main": 0.0, "frontier": 0.0}
             self.jsonl = self.links = self.lane_out = self.lane_in = 0
-            self.upload_s = 0.0
+            self.upload_s = self.dump_s = 0.0
 
         def add(self, r):
             self.launches += r.gpu_launches
@@ -377,7 +451,12 @@ def main():
             self.jsonl += r.jsonl_len; self.links += r.n_links
             self.lane_out += r.main_bytes_out; self.lane_in += r.main_bytes_in
 
-    def step_resident(acc=None):
+    def sample(acc, dump, slot, r):
+        t_d = time.perf_counter()
+        dump.run(slot, r)
+        acc.dump_s += time.perf_counter() - t_d
+
+    def step_resident(acc=None, dump=None):
         eng.frontier_clear()
         r = None
         if is_yt:
@@ -389,11 +468,15 @@ def main():
                 r = eng.youtube_run_resident(0, RUN | abi.RUN_NO_D2H)
                 if acc:
                     acc.add(r)
+                if dump:
+                    sample(acc, dump, 0, r)
         else:
             for i in range(len(corpora)):
                 r = eng.telegram_run_resident(i, RUN | abi.RUN_NO_D2H)
                 if acc:
                     acc.add(r)
+                if dump:
+                    sample(acc, dump, i, r)
         gsize = r.frontier_size
         if merger:
             gsize = merger.merge()
@@ -405,12 +488,20 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     acc = Acc()
+    dump = OutputDump(eng, len(corpora)) if args.dump_outputs else None
     t0 = time.perf_counter()
-    for _ in range(args.steps):
-        gsize = step_resident(acc)
+    for i in range(args.steps):
+        gsize = step_resident(acc, dump if i == args.steps - 1 else None)
     barrier()
-    dt = time.perf_counter() - t0 - acc.upload_s   # YouTube: the uploads between resident batches are not part of `value`
+    # YouTube: the uploads between resident batches are not part of `value`; nor is the sampling of --dump-outputs
+    dt = time.perf_counter() - t0 - acc.upload_s - acc.dump_s
     clocks = sampler.stop()
+    dump_bytes = None
+    if dump:
+        keys = merger.global_export() if merger else eng.frontier_export()  # the merged set's export is collective
+        if rank == 0:
+            dump_bytes = dump.write(args.dump_outputs, keys)
+        del keys
     dt_t = torch.tensor([dt], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(dt_t, op=dist.ReduceOp.MAX)
@@ -462,7 +553,7 @@ def main():
         for _ in range(2):
             d2h_bytes = step_e2e()
         barrier()
-        e2e_steps = max(1, min(args.steps, 3))
+        e2e_steps = args.steps
         t0 = time.perf_counter()
         for _ in range(e2e_steps):
             d2h_bytes = step_e2e()
@@ -552,7 +643,8 @@ def main():
                        "jsonl_bytes_per_gpu": jsonl_len, "links_per_gpu": n_links,
                        "l2": "inputs (%.1f GB) and outputs (%.1f GB) per step are far larger than the 126 MB L2" % (in_bytes / 1e9, jsonl_len / 1e9),
                        "timing": "wall clock around the K steps between barriers + synchronize, max over ranks"
-                                 + ("; host->device uploads between the resident YouTube batches excluded" if is_yt else ""),
+                                 + ("; host->device uploads between the resident YouTube batches excluded" if is_yt else "")
+                                 + ("; sampling of the last step's outputs excluded" if dump else ""),
                        "parallelism": f"record-index sharding x{world}" + ("; NCCL set merge per step: " + merger.describe() if merger else ""),
                        "frontier_unique": int(gsize), "corpus_gen_s": round(t_gen, 2)},
             "clocks": clocks,
@@ -564,6 +656,8 @@ def main():
         }
         if merge_stats:
             line["merge"] = merge_stats
+        if dump:
+            line["dumped_outputs"] = {"dir": args.dump_outputs, "bytes": dump_bytes}
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
