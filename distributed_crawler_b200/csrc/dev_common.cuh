@@ -14,6 +14,20 @@
 
 namespace tgi {
 
+// Error bits the kernels atomicOr into a batch's error word, and the layout of the batch's scalars block (u64 words,
+// zeroed before the batch; the host reads it back).  SC_CURSOR holds the link-arena cursor (u32) and the error word (int).
+enum : int {
+  ERR_ARENA_OVERFLOW = 1,
+  ERR_TOO_MANY_REACTIONS = 2,
+  ERR_FRONTIER_FULL = 4,
+  ERR_TOO_MANY_LINKS = 8,
+  ERR_LINE_MISMATCH = 16,  // sized and emitted line lengths disagree: never expected
+  ERR_PAGE_OVERFLOW = 64,  // a page does not fit its result block: the host reruns it on the bulk pipeline
+  SC_CHAN_TOTAL = 0, SC_LINE_TOTAL = 1, SC_CURSOR = 2, SC_NEW = 3, SC_FSIZE = 4, SC_LINK_TOTAL = 5, SC_LONG = 6,
+  SC_URL_CURSOR = 7, SC_LANE_OUT = 8, SC_LANE_IN = 9, SC_LISTS = 10 /* 3 x u32 */, SC_COUNT = 12,
+  PAGE_TRACE_AT = 16,  // page kernels: phase clock and slowest records behind the scalars (TGI_PAGE_TRACE)
+};
+
 DEVI int lane_id() { return (int)(threadIdx.x & 31); }
 
 // ---- global byte / word loads (read-only path) ---------------------------------------------------

@@ -9,7 +9,6 @@
 //   frontier_*                             exact open-addressed hash set over 32-byte keys
 //   yt_* / gm_*                            YouTube (config 4) and generic-message (a12) lines
 //   join_*                                 message-status join (SURVEY 8f)
-// yt_size_kernel is the warp-per-record predecessor of the YouTube lane sizer, kept as an A/B reference (TGI_YT_WARP).
 #pragma once
 #include "tg_walk.cuh"
 #include "tg_lane.cuh"
@@ -40,47 +39,54 @@ constexpr int CTA_THREADS = WARPS_PER_CTA * 32;
 #define LB_YT 6  // 3: 22.8 ms per 2 M config-4 records, 4: 20.4, 5: 19.2, 6: 18.7, 8: 18.6 (tools/variants_yt.sh)
 #endif
 
-#define ERR_ARENA_OVERFLOW 1
-#define ERR_TOO_MANY_REACTIONS 2
-#define ERR_FRONTIER_FULL 4
-#define ERR_TOO_MANY_LINKS 8
-
 // ---- batch validation: every offset the kernels will follow stays inside its array ------------------------------
 // A malformed batch that crossed the C ABI must come back as TGI_E_ARG, not as an illegal address (or as foreign
-// bytes in the JSONL).  One thread per index of the longest array; big batches only (small ones are checked by the host).
+// bytes in the JSONL).  One rule per element, shared by the host (small batches, host pointers in the TgBatchDev) and
+// tg_validate_kernel (big ones); the result is a mask of the broken checks.
 struct TgBounds {
   uint64_t strs_len, n_ents, n_reacts, n_comments, aux_len, chan_strs_len;
 };
+#define HDI __host__ __device__ __forceinline__
+HDI int tg_check_record(const TgBatchDev& b, const TgBounds& lim, uint64_t i) {
+  const tgi_tg_rec rc = b.recs[i];
+  const uint64_t end = rc.str_off + (uint64_t)rc.text_len + rc.alt_len + rc.media_len + rc.handle_len;
+  int e = 0;
+  if (end > lim.strs_len || end < rc.str_off) e |= 1;
+  if (rc.chan_idx >= b.n_chans || rc.content_type >= TGI_CT__COUNT) e |= 2;
+  if (b.ent_off[i] > b.ent_off[i + 1] || b.ent_off[i + 1] > lim.n_ents) e |= 4;
+  if (b.react_off[i] > b.react_off[i + 1] || b.react_off[i + 1] > lim.n_reacts) e |= 8;
+  if (b.comment_off[i] > b.comment_off[i + 1] || b.comment_off[i + 1] > lim.n_comments) e |= 16;
+  return e;
+}
+HDI int tg_check_entity(const TgBatchDev& b, const TgBounds& lim, uint64_t i) {
+  const tgi_entity en = b.ents[i];
+  return en.type == TGI_ENT_TEXT_URL && (uint64_t)en.url_off + en.url_len > lim.aux_len ? 32 : 0;
+}
+HDI int tg_check_reaction(const TgBatchDev& b, const TgBounds& lim, uint64_t i) {
+  const tgi_reaction rc = b.reacts[i];
+  return (uint64_t)rc.emoji_off + rc.emoji_len > lim.aux_len ? 64 : 0;
+}
+HDI int tg_check_comment(const TgBatchDev& b, const TgBounds& lim, uint64_t i) {
+  const tgi_comment cm = b.comments[i];
+  int e = 0;
+  if ((uint64_t)cm.text_off + cm.text_len > lim.aux_len || (uint64_t)cm.handle_off + cm.handle_len > lim.aux_len) e |= 128;
+  if ((cm.flags & 1) && (uint64_t)cm.react_start + cm.react_count > lim.n_reacts) e |= 256;
+  return e;
+}
+HDI int tg_check_channel(const TgBatchDev& b, const TgBounds& lim, uint64_t i) {
+  const tgi_tg_chan ch = b.chans[i];
+  return (uint64_t)ch.str_off + ch.title_len + ch.name_len + ch.user_len > lim.chan_strs_len ? 512 : 0;
+}
+// one thread per index of the longest array
 __global__ void tg_validate_kernel(TgBatchDev b, TgBounds lim, uint64_t count, int* bad) {
   const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= count) return;
   int e = 0;
-  if (i < b.n) {
-    const tgi_tg_rec rc = b.recs[i];
-    const uint64_t end = rc.str_off + (uint64_t)rc.text_len + rc.alt_len + rc.media_len + rc.handle_len;
-    if (end > lim.strs_len || end < rc.str_off) e |= 1;
-    if (rc.chan_idx >= b.n_chans || rc.content_type >= TGI_CT__COUNT) e |= 2;
-    if (b.ent_off[i] > b.ent_off[i + 1] || b.ent_off[i + 1] > lim.n_ents) e |= 4;
-    if (b.react_off[i] > b.react_off[i + 1] || b.react_off[i + 1] > lim.n_reacts) e |= 8;
-    if (b.comment_off[i] > b.comment_off[i + 1] || b.comment_off[i + 1] > lim.n_comments) e |= 16;
-  }
-  if (i < lim.n_ents) {
-    const tgi_entity en = b.ents[i];
-    if (en.type == TGI_ENT_TEXT_URL && (uint64_t)en.url_off + en.url_len > lim.aux_len) e |= 32;
-  }
-  if (i < lim.n_reacts) {
-    const tgi_reaction rc = b.reacts[i];
-    if ((uint64_t)rc.emoji_off + rc.emoji_len > lim.aux_len) e |= 64;
-  }
-  if (i < lim.n_comments) {
-    const tgi_comment cm = b.comments[i];
-    if ((uint64_t)cm.text_off + cm.text_len > lim.aux_len || (uint64_t)cm.handle_off + cm.handle_len > lim.aux_len) e |= 128;
-    if ((cm.flags & 1) && (uint64_t)cm.react_start + cm.react_count > lim.n_reacts) e |= 256;
-  }
-  if (i < b.n_chans) {
-    const tgi_tg_chan ch = b.chans[i];
-    if ((uint64_t)ch.str_off + ch.title_len + ch.name_len + ch.user_len > lim.chan_strs_len) e |= 512;
-  }
+  if (i < b.n) e |= tg_check_record(b, lim, i);
+  if (i < lim.n_ents) e |= tg_check_entity(b, lim, i);
+  if (i < lim.n_reacts) e |= tg_check_reaction(b, lim, i);
+  if (i < lim.n_comments) e |= tg_check_comment(b, lim, i);
+  if (i < b.n_chans) e |= tg_check_channel(b, lim, i);
   if (e) atomicOr(bad, e);
 }
 
@@ -577,7 +583,7 @@ DEVI void yt_parse_body(const YtBatchDev& b, const CfgDev& cfg, uint32_t run_fla
 }
 __global__ void __launch_bounds__(CTA_THREADS, LB_YT) yt_parse_kernel(YtBatchDev b, CfgDev cfg, uint32_t run_flags, YtOut o) { yt_parse_body(b, cfg, run_flags, o); }
 
-// one record by one warp (yt_size_kernel, yt_page_kernel)
+// one record by one warp (yt_page_kernel)
 DEVI void yt_size_record(const YtBatchDev& b, const CfgDev& cfg, const YtOut& o, uint64_t r, YtScratch* sc) {
   const int l = lane_id();
   {
@@ -605,16 +611,6 @@ DEVI void yt_size_record(const YtBatchDev& b, const CfgDev& cfg, const YtOut& o,
     }
   }
 }
-__global__ void __launch_bounds__(CTA_THREADS, LB_YT) yt_size_kernel(YtBatchDev b, CfgDev cfg, YtOut o) {
-  __shared__ YtScratch scs[WARPS_PER_CTA];
-  int wid = threadIdx.x >> 5;
-  uint64_t nwarps = (uint64_t)gridDim.x * WARPS_PER_CTA;
-  for (uint64_t r = (uint64_t)blockIdx.x * WARPS_PER_CTA + wid; r < b.n; r += nwarps) {
-    if (o.status[r] != TGI_ST_EMITTED) continue;  // linelen stays 0
-    yt_size_record(b, cfg, o, r, &scs[wid]);
-  }
-}
-
 // length pass, one lane per record (yt_lane.cuh); the description and the title are measured by the warp
 __global__ void __launch_bounds__(CTA_THREADS, LB_YT) yt_size_lane_kernel(YtBatchDev b, CfgDev cfg, YtOut o) {
   const int wid = threadIdx.x >> 5, l = lane_id();
@@ -664,7 +660,7 @@ __global__ void __launch_bounds__(CTA_THREADS, LB_YT) yt_size_lane_kernel(YtBatc
 }
 
 // warp writer: the records the lane writer does not take (a string needs escaping); lanes pick them out of
-// groups of 32.  lane_mode == 0: every record (A/B reference, TGI_YT_WARP=1).
+// groups of 32.  yt_page_kernel writes every record with yt_emit_record.
 DEVI void yt_emit_record(const YtBatchDev& b, const CfgDev& cfg, const YtOut& o, const uint64_t* line_off, uint8_t* out, int* err,
                          uint64_t r, YtScratch* sc) {
   YtArgs a;
@@ -679,17 +675,16 @@ DEVI void yt_emit_record(const YtBatchDev& b, const CfgDev& cfg, const YtOut& o,
   w.el[1] = o.esc_len[3 * r + 1];
   w.p = out + line_off[r];
   walk_yt_record(w, a);
-  if (lane_id() == 0 && (uint64_t)(w.p - out) != line_off[r + 1]) atomicOr(err, 16);
+  if (lane_id() == 0 && (uint64_t)(w.p - out) != line_off[r + 1]) atomicOr(err, ERR_LINE_MISMATCH);
   __syncwarp();
 }
-__global__ void __launch_bounds__(CTA_THREADS, LB_YT) yt_emit_kernel(YtBatchDev b, CfgDev cfg, YtOut o, const uint64_t* line_off, uint8_t* out, int* err,
-                                                                 int lane_mode) {
+__global__ void __launch_bounds__(CTA_THREADS, LB_YT) yt_emit_kernel(YtBatchDev b, CfgDev cfg, YtOut o, const uint64_t* line_off, uint8_t* out, int* err) {
   __shared__ YtScratch scs[WARPS_PER_CTA];
   int wid = threadIdx.x >> 5, l = lane_id();
   const uint64_t ngroups = (b.n + 31) / 32, nwarps = (uint64_t)gridDim.x * WARPS_PER_CTA;
   for (uint64_t g = (uint64_t)blockIdx.x * WARPS_PER_CTA + wid; g < ngroups; g += nwarps) {
     const uint64_t rl = g * 32 + l;
-    uint32_t todo = __ballot_sync(FULL, rl < b.n && o.status[rl] == TGI_ST_EMITTED && !(lane_mode && o.esc_len[3 * rl + 2]));
+    uint32_t todo = __ballot_sync(FULL, rl < b.n && o.status[rl] == TGI_ST_EMITTED && !o.esc_len[3 * rl + 2]);
     while (todo) {
       const uint64_t r = g * 32 + (uint32_t)(__ffs(todo) - 1);
       todo &= todo - 1;
@@ -718,7 +713,7 @@ __global__ void __launch_bounds__(CTA_THREADS, LB_YT) yt_emit_lane_kernel(YtBatc
       w.begin((uint64_t)(uintptr_t)out + line_off[r]);
       walk_yt_record(w, a);
       w.end();
-      if (w.s.pos != (uint64_t)(uintptr_t)out + line_off[r + 1]) atomicOr(err, 16);
+      if (w.s.pos != (uint64_t)(uintptr_t)out + line_off[r + 1]) atomicOr(err, ERR_LINE_MISMATCH);
     }
     __syncwarp();
     w.flush_pending(active);
@@ -790,7 +785,7 @@ __global__ void __launch_bounds__(CTA_THREADS, 4) gm_emit_kernel(GmBatchDev b, C
     w.sc = &scs[wid];
     w.p = out + line_off[r];
     walk_gm_record(w, b, cfg, r);
-    if (l == 0 && (uint64_t)(w.p - out) != line_off[r + 1]) atomicOr(err, 16);
+    if (l == 0 && (uint64_t)(w.p - out) != line_off[r + 1]) atomicOr(err, ERR_LINE_MISMATCH);
   }
 }
 

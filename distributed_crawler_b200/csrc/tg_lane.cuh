@@ -442,7 +442,7 @@ DEVI void emit_tg_lane(LaneShared& sh, uint32_t* row, LaneStream& s, const TgBat
   ls_flush(s);
   ls_drain_warp(s);
   if (active) {
-    if ((uint32_t)(s.pos - line_start) != total) atomicOr(err, 16);  // sizing and emission disagree: never expected
+    if ((uint32_t)(s.pos - line_start) != total) atomicOr(err, ERR_LINE_MISMATCH);
     bytes_out += total - gaps;
     bytes_in += copied;
   }

@@ -28,8 +28,7 @@
 namespace tgi {
 namespace cg = cooperative_groups;
 
-#define ERR_PAGE_OVERFLOW 64
-constexpr int PAGE_TRACE_AT = 16, PAGE_PHASES = 7;  // scalars[16 .. 16 + 8): start, after each barrier, end
+constexpr int PAGE_PHASES = 7;  // scalars[PAGE_TRACE_AT .. + 8): start, after each barrier, end
 
 struct PageArgs {
   TgBatchDev b;
@@ -57,8 +56,6 @@ struct PageArgs {
   ExclusionDev excl;
   uint64_t bslots;
   uint64_t* new_off;       // [n+1]
-  // indices into `scalars`
-  int sc_chan_total, sc_line_total, sc_link_total, sc_new, sc_count;
 };
 
 // exclusive scan u32[n] -> u64[n+1] by ONE CTA of CTA_THREADS threads (all of them call it)
@@ -139,7 +136,7 @@ __global__ void __launch_bounds__(CTA_THREADS, 2) tg_page_kernel(const __grid_co
   if (blockIdx.x == 0 && threadIdx.x < 3) a.scalars[PAGE_TRACE_AT + PAGE_PHASES + 1 + threadIdx.x] = 0;
 
   // P0
-  if (blockIdx.x == 0 && (int)threadIdx.x < a.sc_count) a.scalars[threadIdx.x] = 0;
+  if (blockIdx.x == 0 && threadIdx.x < SC_COUNT) a.scalars[threadIdx.x] = 0;
   if (want_fr) grid_zero16(a.fb.btable, a.bslots * 8);
   if (want_json) {
     grid_zero16(a.chan_blob, a.chan_blob_cap);  // segment padding must read as zero
@@ -167,14 +164,14 @@ __global__ void __launch_bounds__(CTA_THREADS, 2) tg_page_kernel(const __grid_co
     slowest(0, tb, r);
   }
   if (want_json && blockIdx.x == last) {
-    cta_scan_u32(a.chan_len, a.b.n_chans, a.chan_off, a.scalars + a.sc_chan_total);
+    cta_scan_u32(a.chan_len, a.b.n_chans, a.chan_off, a.scalars + SC_CHAN_TOTAL);
     __syncthreads();
     for (uint32_t c = threadIdx.x; c < a.b.n_chans; c += blockDim.x) a.chan_derived[c].off = a.chan_off[c];
   }
   grid.sync();
   stamp();
   if (*(volatile int*)a.po.err & (ERR_ARENA_OVERFLOW | ERR_TOO_MANY_LINKS)) return;  // the host reruns the ordinary pipeline
-  if (want_json && a.scalars[a.sc_chan_total] > a.chan_blob_cap) {
+  if (want_json && a.scalars[SC_CHAN_TOTAL] > a.chan_blob_cap) {
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(a.po.err, ERR_PAGE_OVERFLOW);
     return;
   }
@@ -215,20 +212,20 @@ __global__ void __launch_bounds__(CTA_THREADS, 2) tg_page_kernel(const __grid_co
   stamp();
 
   // P3
-  if (want_json && blockIdx.x == 0) cta_scan_u32(a.po.linelen, n, a.line_off, a.scalars + a.sc_line_total);
-  if (want_links && blockIdx.x == 1 % gridDim.x) cta_scan_u32(a.po.link_count, n, a.link_off, a.scalars + a.sc_link_total);
+  if (want_json && blockIdx.x == 0) cta_scan_u32(a.po.linelen, n, a.line_off, a.scalars + SC_LINE_TOTAL);
+  if (want_links && blockIdx.x == 1 % gridDim.x) cta_scan_u32(a.po.link_count, n, a.link_off, a.scalars + SC_LINK_TOTAL);
   if (want_fr) frontier_count_body(n, a.po.link_start, a.po.link_count, a.fb, t0, nt);
   grid.sync();
   stamp();
 
   // P4
   if (want_fr) {
-    if (blockIdx.x == last) cta_scan_u32(a.fb.rec_new, n, a.new_off, a.scalars + a.sc_new);
+    if (blockIdx.x == last) cta_scan_u32(a.fb.rec_new, n, a.new_off, a.scalars + SC_NEW);
     grid.sync();
   }
   stamp();
-  const uint64_t links_bytes = want_links ? (a.scalars[a.sc_link_total] * sizeof(tgi_link) + 255) & ~255ull : 0;
-  const uint64_t line_total = want_json ? a.scalars[a.sc_line_total] : 0;
+  const uint64_t links_bytes = want_links ? (a.scalars[SC_LINK_TOTAL] * sizeof(tgi_link) + 255) & ~255ull : 0;
+  const uint64_t line_total = want_json ? a.scalars[SC_LINE_TOTAL] : 0;
   if (links_bytes + line_total > a.var_cap || (a.max_out && line_total > a.max_out)) {
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(a.po.err, ERR_PAGE_OVERFLOW);
     return;
@@ -273,7 +270,7 @@ __global__ void __launch_bounds__(CTA_THREADS, 2) tg_page_kernel(const __grid_co
 
   // P6
   if (want_links) links_compact_body(n, a.po.link_start, a.po.link_count, a.link_off, a.po.arena, (tgi_link*)a.var, a.link_off32);
-  if (want_fr && blockIdx.x == last && threadIdx.x == 0) frontier_commit_body(a.fr, a.new_off, n, a.scalars + a.sc_new, a.po.err);
+  if (want_fr && blockIdx.x == last && threadIdx.x == 0) frontier_commit_body(a.fr, a.new_off, n, a.scalars + SC_NEW, a.po.err);
   stamp();  // block 0's own end of P6
 }
 

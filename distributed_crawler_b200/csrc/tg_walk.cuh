@@ -599,8 +599,8 @@ DEVI void emit_tg_fixed(uint8_t* line, WarpScratch* ws, const CtaShared* cs, con
     off[k] = run;
     run += len[k];
   }
-  if (__shfl_sync(FULL, incl, 31) != total) {  // sizing and emission disagree: never expected; the host reports it
-    if (l == 0) atomicOr(err, 16);
+  if (__shfl_sync(FULL, incl, 31) != total) {  // the host reports it
+    if (l == 0) atomicOr(err, ERR_LINE_MISMATCH);
     return;
   }
 #pragma unroll

@@ -117,6 +117,7 @@ struct Slot {
   uint32_t page_bpr = 3072;              // running estimate of result bytes per record (sizes the speculative read)
   const uint8_t* dev_jsonl = nullptr;    // where the last batch's JSONL lives on the device (tgi_result_read_jsonl)
   // resident batch descriptor
+  JobKind batch = JOB_NONE;  // the kind of the last uploaded batch: JOB_TG, JOB_YT or JOB_GM
   TgBatchDev tg{};
   YtBatchDev yt{};
   GmBatchDev gm{};
@@ -126,7 +127,7 @@ struct Slot {
   uint64_t dev_jsonl_len = 0;
   // what tgi_pending_edges needs from the slot's last batch
   uint64_t last_n = 0, last_new = 0;
-  bool last_frontier = false, last_yt = false;
+  bool last_frontier = false;
   // job hand-off
   std::mutex mu;
   std::condition_variable cv;
@@ -349,9 +350,7 @@ int launch_scan(tgi_ctx* c, Slot& s, const uint32_t* in, uint64_t n, uint64_t* o
   return TGI_OK;
 }
 
-template <class T>
-int h2d(tgi_ctx* c, Slot& s, DevBuf& d, const T* src, size_t count) {
-  size_t bytes = count * sizeof(T);
+int h2d(tgi_ctx* c, Slot& s, DevBuf& d, const void* src, size_t bytes) {
   cudaStream_t st = s.stream;
   CK(d.ensure(bytes));
   if (bytes) CK(cudaMemcpyAsync(d.p, src, bytes, cudaMemcpyHostToDevice, st));
@@ -378,36 +377,17 @@ int publish(tgi_ctx* c, const void* d_src, HostBuf& h, int n_words, cudaStream_t
   return TGI_OK;
 }
 
-enum { SC_CHAN_TOTAL = 0, SC_LINE_TOTAL = 1, SC_CURSOR = 2, SC_NEW = 3, SC_FSIZE = 4, SC_LINK_TOTAL = 5, SC_LONG = 6, SC_URL_CURSOR = 7, SC_LANE_OUT = 8, SC_LANE_IN = 9, SC_LISTS = 10 /* 3 x u32 */, SC_COUNT = 12 };
 constexpr uint64_t HOST_VALIDATE_MAX = 1u << 16;  // batches up to this many elements are range-checked on the host
 
 // the checks of tg_validate_kernel, on the host (small batches: no extra launch / sync in a page-sized call)
-int host_validate_tg(const tgi_tg_batch* in) {
-  const uint64_t n = in->n, n_ents = n ? in->ent_off[n] : 0;
+int host_validate_tg(const TgBatchDev& b, const TgBounds& lim) {
   int e = 0;
-  for (uint64_t i = 0; i < n; i++) {
-    const tgi_tg_rec& rc = in->recs[i];
-    const uint64_t end = rc.str_off + (uint64_t)rc.text_len + rc.alt_len + rc.media_len + rc.handle_len;
-    if (end > in->strs_len || end < rc.str_off) e |= 1;
-    if (rc.chan_idx >= in->n_chans || rc.content_type >= TGI_CT__COUNT) e |= 2;
-    if (in->ent_off[i] > in->ent_off[i + 1]) e |= 4;
-    if (in->react_off[i] > in->react_off[i + 1] || in->react_off[i + 1] > in->n_reacts) e |= 8;
-    if (in->comment_off[i] > in->comment_off[i + 1] || in->comment_off[i + 1] > in->n_comments) e |= 16;
-  }
+  for (uint64_t i = 0; i < b.n; i++) e |= tg_check_record(b, lim, i);
   if (e) return e;  // the entity count itself comes from ent_off: do not follow it if the offsets are broken
-  for (uint64_t i = 0; i < n_ents; i++)
-    if (in->ents[i].type == TGI_ENT_TEXT_URL && (uint64_t)in->ents[i].url_off + in->ents[i].url_len > in->aux_len) e |= 32;
-  for (uint64_t i = 0; i < in->n_reacts; i++)
-    if ((uint64_t)in->reacts[i].emoji_off + in->reacts[i].emoji_len > in->aux_len) e |= 64;
-  for (uint64_t i = 0; i < in->n_comments; i++) {
-    const tgi_comment& cm = in->comments[i];
-    if ((uint64_t)cm.text_off + cm.text_len > in->aux_len || (uint64_t)cm.handle_off + cm.handle_len > in->aux_len) e |= 128;
-    if ((cm.flags & 1) && (uint64_t)cm.react_start + cm.react_count > in->n_reacts) e |= 256;
-  }
-  for (uint32_t i = 0; i < in->n_chans; i++) {
-    const tgi_tg_chan& ch = in->chans[i];
-    if ((uint64_t)ch.str_off + ch.title_len + ch.name_len + ch.user_len > in->chan_strs_len) e |= 512;
-  }
+  for (uint64_t i = 0; i < lim.n_ents; i++) e |= tg_check_entity(b, lim, i);
+  for (uint64_t i = 0; i < lim.n_reacts; i++) e |= tg_check_reaction(b, lim, i);
+  for (uint64_t i = 0; i < lim.n_comments; i++) e |= tg_check_comment(b, lim, i);
+  for (uint32_t i = 0; i < b.n_chans; i++) e |= tg_check_channel(b, lim, i);
   return e;
 }
 
@@ -428,10 +408,6 @@ int validate_tg(tgi_ctx* c, const tgi_tg_batch* in) {
     set_err(c, "telegram batch: a non-empty array has a null pointer");
     return TGI_E_ARG;
   }
-  if (in->n + n_ents + in->n_reacts + in->n_comments + in->n_chans <= HOST_VALIDATE_MAX) {
-    const int e = host_validate_tg(in);
-    if (e) { set_err(c, "telegram batch: offsets outside their arrays (mask 0x%x)", e); return TGI_E_ARG; }
-  }
   return TGI_OK;
 }
 
@@ -446,129 +422,118 @@ unsigned grid_mult() {
   return v;
 }
 
-// ---- page-sized batches: one block in, one launch, one block out (tg_page.cuh) ---------------------------------------
+// ---- page-sized batches: one block in, one launch, one block out (tg_page.cuh, yt_page.cuh) -------------------------
 constexpr uint64_t PAGE_MAX_RECS = 8192;          // the in-kernel scans are single-CTA
 constexpr uint64_t PAGE_MAX_IN_BYTES = 4u << 20;
-bool page_enabled() {
-  return getenv("TGI_NO_PAGE") == nullptr;  // A/B switch (read per call): the ordinary pipeline for every size
+// Which batches take the page kernels.  At upload, page_sized(packed size) selects the one-block upload; at run time,
+// page_run (the sizes of the resident batch and the run flags) selects the page kernel.
+bool page_sized(uint64_t n, uint32_t n_chans, uint64_t in_bytes) {
+  if (getenv("TGI_NO_PAGE")) return false;  // A/B switch (read per call): the ordinary pipeline for every size
+  return n && n <= PAGE_MAX_RECS && n_chans <= PAGE_MAX_RECS && in_bytes <= PAGE_MAX_IN_BYTES;
 }
-struct PageInLayout {
-  size_t off[11], bytes[11], total;
-};
-PageInLayout page_in_layout(const tgi_tg_batch* in, uint64_t n_ents) {
-  const uint64_t n = in->n;
-  const size_t b[11] = {n * sizeof(tgi_tg_rec), in->strs_len, (n + 1) * 4, n_ents * sizeof(tgi_entity), (n + 1) * 4,
-                        in->n_reacts * sizeof(tgi_reaction), (n + 1) * 4, in->n_comments * sizeof(tgi_comment), in->aux_len,
-                        in->n_chans * sizeof(tgi_tg_chan), in->chan_strs_len};
-  PageInLayout L;
-  size_t o = 0;
-  for (int i = 0; i < 11; i++) {
-    L.off[i] = o;
-    L.bytes[i] = b[i];
-    o += (b[i] + PAD + 15) & ~(size_t)15;  // PAD readable zero bytes behind every array, as h2d() leaves them
-  }
-  L.total = o;
-  return L;
-}
-bool page_sized(const tgi_tg_batch* in, uint64_t n_ents) {
-  if (!page_enabled() || in->n == 0 || in->n > PAGE_MAX_RECS || in->n_chans > PAGE_MAX_RECS) return false;
-  if (in->n + n_ents + in->n_reacts + in->n_comments + in->n_chans > HOST_VALIDATE_MAX) return false;  // validate_tg checked every offset
-  return page_in_layout(in, n_ents).total <= PAGE_MAX_IN_BYTES;
+bool page_run(const Slot& s, uint64_t n, uint32_t n_chans, uint32_t flags) {
+  if (!page_sized(n, n_chans, s.in_bytes)) return false;
+  if (flags & TGI_RUN_NO_D2H) return false;  // a device-resident result keeps the ordinary buffers
+  return (flags & (TGI_RUN_JSONL | TGI_RUN_LINKS | TGI_RUN_FRONTIER)) != 0;
 }
 
-// The eleven input arrays packed into one pinned block and sent with ONE copy (eleven copies + eleven pad memsets are a
-// third of what a 100-message call costs otherwise).  The pack is a host memcpy of the page (tens of KB).
-int upload_tg_page(tgi_ctx* c, Slot& s, const tgi_tg_batch* in, uint64_t n_ents) {
-  const uint64_t n = in->n;
-  const PageInLayout L = page_in_layout(in, n_ents);
-  CK(s.h_page_in.ensure(L.total));
-  CK(s.d_page_in.ensure(L.total));
-  uint8_t* h = s.h_page_in.as<uint8_t>();
-  const void* src[11] = {in->recs, in->strs, in->ent_off, in->ents, in->react_off, in->reacts, in->comment_off, in->comments,
-                         in->aux, in->chans, in->chan_strs};
-  for (int i = 0; i < 11; i++) {
-    if (L.bytes[i]) memcpy(h + L.off[i], src[i], L.bytes[i]);
-    const size_t end = i + 1 < 11 ? L.off[i + 1] : L.total;
-    memset(h + L.off[i] + L.bytes[i], 0, end - L.off[i] - L.bytes[i]);
+// One input array of a batch: the slot buffer it goes to when sent on its own, where it comes from, its size.
+struct InArray {
+  DevBuf* buf;
+  const void* src;
+  size_t bytes;
+};
+size_t packed_bytes(const InArray& a) { return (a.bytes + PAD + 15) & ~(size_t)15; }  // PAD zero bytes behind, as h2d() leaves them
+size_t packed_size(const InArray* a, int k) {
+  size_t t = 0;
+  for (int i = 0; i < k; i++) t += packed_bytes(a[i]);
+  return t;
+}
+// Sends a batch's input arrays and stores their device addresses in dev[].  packed: all of them in one pinned block and
+// ONE copy (for a page, eleven copies and eleven pads are a third of what a 100-message call costs; the pack is a host
+// memcpy of tens of KB).  Otherwise one copy per array into its slot buffer.
+int upload_arrays(tgi_ctx* c, Slot& s, const InArray* a, int k, bool packed, const uint8_t** dev) {
+  s.in_bytes = 0;
+  if (!packed) {
+    for (int i = 0; i < k; i++) {
+      const int rc = h2d(c, s, *a[i].buf, a[i].src, a[i].bytes);
+      if (rc) return rc;
+      dev[i] = a[i].buf->as<uint8_t>();
+    }
+    return TGI_OK;
   }
-  CK(cudaMemcpyAsync(s.d_page_in.p, h, L.total, cudaMemcpyHostToDevice, s.stream));
-  uint8_t* d = s.d_page_in.as<uint8_t>();
-  TgBatchDev& b = s.tg;
-  b.n = n;
-  b.recs = (const tgi_tg_rec*)(d + L.off[0]);
-  b.strs = d + L.off[1];
-  b.ent_off = (const uint32_t*)(d + L.off[2]);
-  b.ents = (const tgi_entity*)(d + L.off[3]);
-  b.react_off = (const uint32_t*)(d + L.off[4]);
-  b.reacts = (const tgi_reaction*)(d + L.off[5]);
-  b.comment_off = (const uint32_t*)(d + L.off[6]);
-  b.comments = (const tgi_comment*)(d + L.off[7]);
-  b.aux = d + L.off[8];
-  b.n_chans = in->n_chans;
-  b.chans = (const tgi_tg_chan*)(d + L.off[9]);
-  b.chan_strs = d + L.off[10];
-  s.n_ents = n_ents;
-  s.n_reacts = in->n_reacts;
-  s.n_comments = in->n_comments;
-  s.chan_strs_len = in->chan_strs_len;
-  for (int i = 0; i < 11; i++) s.in_bytes += L.bytes[i];
-  s.resident = true;  // the element count is below HOST_VALIDATE_MAX: validate_tg has range-checked every offset
+  const size_t total = packed_size(a, k);
+  CK(s.h_page_in.ensure(total));
+  CK(s.d_page_in.ensure(total));
+  uint8_t* h = s.h_page_in.as<uint8_t>();
+  size_t o = 0;
+  for (int i = 0; i < k; i++) {
+    if (a[i].bytes) memcpy(h + o, a[i].src, a[i].bytes);
+    memset(h + o + a[i].bytes, 0, packed_bytes(a[i]) - a[i].bytes);
+    dev[i] = s.d_page_in.as<uint8_t>() + o;
+    s.in_bytes += a[i].bytes;
+    o += packed_bytes(a[i]);
+  }
+  CK(cudaMemcpyAsync(s.d_page_in.p, h, total, cudaMemcpyHostToDevice, s.stream));
   return TGI_OK;
 }
 
 int upload_tg(tgi_ctx* c, Slot& s, const tgi_tg_batch* in) {
   int rc = validate_tg(c, in);
   if (rc) return rc;
+  const uint64_t n = in->n, n_ents = n ? in->ent_off[n] : 0;
+  const TgBounds lim{in->strs_len, n_ents, in->n_reacts, in->n_comments, in->aux_len, in->chan_strs_len};
+  const bool host_checked = n + n_ents + in->n_reacts + in->n_comments + in->n_chans <= HOST_VALIDATE_MAX;
+  if (host_checked) {
+    const TgBatchDev hb{n, in->recs, in->strs, in->ent_off, in->ents, in->react_off, in->reacts, in->comment_off, in->comments,
+                        in->aux, in->n_chans, in->chans, in->chan_strs};
+    const int e = host_validate_tg(hb, lim);
+    if (e) { set_err(c, "telegram batch: offsets outside their arrays (mask 0x%x)", e); return TGI_E_ARG; }
+  }
   trace_slot(s, "upload: enqueue");
-  uint64_t n = in->n;
-  s.in_bytes = 0;
-  uint64_t n_ents = n ? in->ent_off[n] : 0;
-  if (page_sized(in, n_ents)) return upload_tg_page(c, s, in, n_ents);
-#define UP(buf, ptr, cnt)                      \
-  rc = h2d(c, s, s.buf, ptr, (size_t)(cnt));   \
+  const InArray arr[11] = {{&s.d_recs, in->recs, n * sizeof(tgi_tg_rec)},
+                           {&s.d_strs, in->strs, in->strs_len},
+                           {&s.d_ent_off, in->ent_off, (n + 1) * 4},
+                           {&s.d_ents, in->ents, n_ents * sizeof(tgi_entity)},
+                           {&s.d_react_off, in->react_off, (n + 1) * 4},
+                           {&s.d_reacts, in->reacts, in->n_reacts * sizeof(tgi_reaction)},
+                           {&s.d_comment_off, in->comment_off, (n + 1) * 4},
+                           {&s.d_comments, in->comments, in->n_comments * sizeof(tgi_comment)},
+                           {&s.d_aux, in->aux, in->aux_len},
+                           {&s.d_chans, in->chans, in->n_chans * sizeof(tgi_tg_chan)},
+                           {&s.d_chan_strs, in->chan_strs, in->chan_strs_len}};
+  const uint8_t* d[11];
+  // a packed page has no device check, so only a batch the host has range-checked is packed
+  rc = upload_arrays(c, s, arr, 11, host_checked && page_sized(n, in->n_chans, packed_size(arr, 11)), d);
   if (rc) return rc;
-  UP(d_recs, in->recs, n);
-  UP(d_strs, in->strs, in->strs_len);
-  UP(d_ent_off, in->ent_off, n + 1);
-  UP(d_ents, in->ents, n_ents);
-  UP(d_react_off, in->react_off, n + 1);
-  UP(d_reacts, in->reacts, in->n_reacts);
-  UP(d_comment_off, in->comment_off, n + 1);
-  UP(d_comments, in->comments, in->n_comments);
-  UP(d_aux, in->aux, in->aux_len);
-  UP(d_chans, in->chans, in->n_chans);
-  UP(d_chan_strs, in->chan_strs, in->chan_strs_len);
-#undef UP
   TgBatchDev& b = s.tg;
   b.n = n;
-  b.recs = s.d_recs.as<tgi_tg_rec>();
-  b.strs = s.d_strs.as<uint8_t>();
-  b.ent_off = s.d_ent_off.as<uint32_t>();
-  b.ents = s.d_ents.as<tgi_entity>();
-  b.react_off = s.d_react_off.as<uint32_t>();
-  b.reacts = s.d_reacts.as<tgi_reaction>();
-  b.comment_off = s.d_comment_off.as<uint32_t>();
-  b.comments = s.d_comments.as<tgi_comment>();
-  b.aux = s.d_aux.as<uint8_t>();
+  b.recs = (const tgi_tg_rec*)d[0];
+  b.strs = d[1];
+  b.ent_off = (const uint32_t*)d[2];
+  b.ents = (const tgi_entity*)d[3];
+  b.react_off = (const uint32_t*)d[4];
+  b.reacts = (const tgi_reaction*)d[5];
+  b.comment_off = (const uint32_t*)d[6];
+  b.comments = (const tgi_comment*)d[7];
+  b.aux = d[8];
   b.n_chans = in->n_chans;
-  b.chans = s.d_chans.as<tgi_tg_chan>();
-  b.chan_strs = s.d_chan_strs.as<uint8_t>();
+  b.chans = (const tgi_tg_chan*)d[9];
+  b.chan_strs = d[10];
   s.n_ents = n_ents;
   s.n_reacts = in->n_reacts;
   s.n_comments = in->n_comments;
   s.chan_strs_len = in->chan_strs_len;
-  if (n + n_ents + in->n_reacts + in->n_comments + in->n_chans > HOST_VALIDATE_MAX) {  // big batch: range-check on the device
+  s.batch = JOB_TG;
+  if (!host_checked) {  // big batch: range-check on the device
     CK(s.d_scalars.ensure(SC_COUNT * 8));
     int* bad = (int*)s.d_scalars.p;
     CK(cudaMemsetAsync(bad, 0, 4, s.stream));
-    TgBounds lim{in->strs_len, n_ents, in->n_reacts, in->n_comments, in->aux_len, in->chan_strs_len};
     const uint64_t count = std::max<uint64_t>({n, n_ents, in->n_reacts, in->n_comments, (uint64_t)in->n_chans});
     tg_validate_kernel<<<(unsigned)((count + 255) / 256), 256, 0, s.stream>>>(b, lim, count, bad);
     CK(s.h_scalars.ensure(SC_COUNT * 8));
-    {
-      const int prc = publish(c, bad, s.h_scalars, 1, s.stream);
-      if (prc) return prc;
-    }
+    rc = publish(c, bad, s.h_scalars, 1, s.stream);
+    if (rc) return rc;
     CK(cudaStreamSynchronize(s.stream));
     const int hbad = *s.h_scalars.as<int>();
     trace_slot(s, "upload: landed + validated");
@@ -611,17 +576,75 @@ void turn_pass(tgi_ctx* c, Slot& s) {
   turn_end(c, s);
 }
 
-// scalars block (device + pinned mirror): [0] chan total, [1] line total, [2] cursor(u32)+err(int),
-// [3] n_new, [4] frontier size, [5] link total
+// Scratch of a batch's frontier phases: the batch hash table (a power of two >= 2 x table_rows entries), one link state
+// per arena row, the new-key count and offset of every record.
+int frontier_scratch(tgi_ctx* c, Slot& s, uint64_t n, uint64_t table_rows, uint64_t arena_cap, FrontierBatch& fb) {
+  const uint64_t bslots = next_pow2(std::max<uint64_t>(2 * table_rows, 1024));
+  CK(s.d_btable.ensure(bslots * 8));
+  CK(s.d_lstate.ensure((size_t)arena_cap * 4));
+  CK(s.d_rec_new.ensure(n * 4));
+  CK(s.d_new_off.ensure((n + 1) * 8));
+  fb.btable = s.d_btable.as<uint64_t>();
+  fb.bmask = bslots - 1;
+  fb.lstate = s.d_lstate.as<uint32_t>();
+  fb.rec_new = s.d_rec_new.as<uint32_t>();
+  return TGI_OK;
+}
 
-// shared tail of the Telegram and YouTube pipelines: frontier phases, link compaction, D2H, result
+// ---- the result: shared by the bulk and the page paths of every batch kind -----------------------------------------------
+// the error bits every path reports the same way once the batch is done
+int device_errors(tgi_ctx* c, int dev_err) {
+  if (dev_err & ERR_FRONTIER_FULL) { set_err(c, "frontier capacity %llu exceeded", (unsigned long long)c->fr.cap); return TGI_E_CAPACITY; }
+  if (dev_err & ERR_LINE_MISMATCH) { set_err(c, "internal: sized and emitted line lengths disagree"); return TGI_E_STATE; }
+  return TGI_OK;
+}
+int check_out_bytes(tgi_ctx* c, uint64_t line_total) {
+  if (c->cfg.max_out_bytes && line_total > c->cfg.max_out_bytes) {
+    set_err(c, "JSONL output %llu bytes exceeds max_out_bytes", (unsigned long long)line_total);
+    return TGI_E_CAPACITY;
+  }
+  return TGI_OK;
+}
+// The fields of a batch's tgi_result that do not depend on the path (out is zeroed by the caller), from the scalars block
+// `hsc` on the host; what tgi_pending_edges needs from the slot's last batch; the context's stats.
+void fill_result(tgi_ctx* c, Slot& s, uint64_t n, uint32_t flags, const uint64_t* hsc, uint64_t line_total, uint64_t n_links,
+                 uint32_t launches, tgi_result* out) {
+  const bool want_json = flags & TGI_RUN_JSONL, want_fr = flags & TGI_RUN_FRONTIER;
+  out->n = n;
+  float ms = 0;
+  cudaEventElapsedTime(&ms, s.ev_k0, s.ev_k1);
+  out->kernel_ms = ms;
+  out->gpu_launches = launches;
+  out->slot = s.idx;
+  if (n && want_json) {
+    out->var_bytes = hsc[SC_LONG];
+    out->main_bytes_out = hsc[SC_LANE_OUT];
+    out->main_bytes_in = hsc[SC_LANE_IN];
+  }
+  out->jsonl_len = want_json ? line_total : 0;
+  out->n_links = n_links;
+  out->n_new = want_fr ? hsc[SC_NEW] : 0;
+  out->frontier_size = want_fr ? hsc[SC_FSIZE] : 0;
+  s.last_n = n;
+  s.last_new = out->n_new;
+  s.last_frontier = want_fr && n;
+  std::lock_guard<std::mutex> g(c->st_mu);
+  c->stats.records += n;
+  c->stats.bytes_in += s.in_bytes;
+  c->stats.bytes_out += out->jsonl_len;
+  c->stats.links += n_links;
+  c->stats.launches += launches;
+  c->stats.kernel_ms_total += ms;
+  if (want_fr) c->stats.frontier_size = out->frontier_size;
+}
+
+// shared tail of the Telegram, YouTube and generic pipelines: frontier phases, link compaction, D2H, result
 int finish_batch(tgi_ctx* c, Slot& s, uint64_t n, uint32_t flags, uint64_t line_total, uint32_t arena_used,
-                 uint64_t arena_cap, uint64_t var_bytes, uint32_t launches, tgi_result* out) {
+                 uint64_t arena_cap, uint32_t launches, tgi_result* out) {
   cudaStream_t st = s.stream;
   const bool want_json = flags & TGI_RUN_JSONL, want_links = flags & TGI_RUN_LINKS, want_fr = flags & TGI_RUN_FRONTIER;
   uint64_t* dsc = s.d_scalars.as<uint64_t>();
   uint64_t* hsc = s.h_scalars.as<uint64_t>();
-  int dev_err = 0;
   s.dev_jsonl_len = want_json ? line_total : 0;
   s.dev_jsonl = s.d_jsonl.as<uint8_t>();
 
@@ -630,24 +653,17 @@ int finish_batch(tgi_ctx* c, Slot& s, uint64_t n, uint32_t flags, uint64_t line_
     turn_begin(c, s);
     std::unique_lock<std::mutex> fg(c->fr_mu);
     if (c->fr_event_valid) CK(cudaStreamWaitEvent(st, c->fr_event, 0));
-    uint64_t bslots = next_pow2(std::max<uint64_t>(2ull * arena_used, 1024));
-    CK(s.d_btable.ensure(bslots * 8));
-    CK(s.d_lstate.ensure((size_t)arena_cap * 4));
-    CK(s.d_rec_new.ensure(n * 4));
-    CK(s.d_new_off.ensure((n + 1) * 8));
-    CK(cudaEventRecord(s.ev_fr0, st));
-    CK(cudaMemsetAsync(s.d_btable.p, 0, bslots * 8, st));
     FrontierBatch fb;
-    fb.btable = s.d_btable.as<uint64_t>();
-    fb.bmask = bslots - 1;
-    fb.lstate = s.d_lstate.as<uint32_t>();
-    fb.rec_new = s.d_rec_new.as<uint32_t>();
+    int rc = frontier_scratch(c, s, n, arena_used, arena_cap, fb);
+    if (rc) return rc;
+    CK(cudaEventRecord(s.ev_fr0, st));
+    CK(cudaMemsetAsync(fb.btable, 0, (fb.bmask + 1) * 8, st));
     unsigned g = (unsigned)((n + 255) / 256);
     frontier_probe_kernel<<<g, 256, 0, st>>>(n, s.d_link_start.as<uint32_t>(), s.d_link_count.as<uint32_t>(),
                                              s.d_arena.as<tgi_link>(), flags, c->fr, fb, c->excl);
     frontier_count_kernel<<<g, 256, 0, st>>>(n, s.d_link_start.as<uint32_t>(), s.d_link_count.as<uint32_t>(), fb);
     launches += 2;
-    int rc = launch_scan(c, s, fb.rec_new, n, s.d_new_off.as<uint64_t>(), dsc + SC_NEW, launches);
+    rc = launch_scan(c, s, fb.rec_new, n, s.d_new_off.as<uint64_t>(), dsc + SC_NEW, launches);
     if (rc) return rc;
     int* derr = (int*)(dsc + SC_CURSOR) + 1;
     frontier_append_kernel<<<g, 256, 0, st>>>(n, s.d_link_start.as<uint32_t>(), s.d_link_count.as<uint32_t>(),
@@ -680,7 +696,6 @@ int finish_batch(tgi_ctx* c, Slot& s, uint64_t n, uint32_t flags, uint64_t line_
   memset(out, 0, sizeof *out);
   out->n = n;
   const bool d2h = !(flags & TGI_RUN_NO_D2H);
-  uint64_t n_links_total = 0;
   if (d2h) {
     CK(s.h_status.ensure(n + 1));
     CK(cudaMemcpyAsync(s.h_status.p, s.d_status.p, n, cudaMemcpyDeviceToHost, st));
@@ -702,33 +717,17 @@ int finish_batch(tgi_ctx* c, Slot& s, uint64_t n, uint32_t flags, uint64_t line_
   trace_slot(s, "emit + frontier + result copy: enqueued");
   CK(cudaStreamSynchronize(st));
   trace_slot(s, "result landed");
-  dev_err = ((int*)(hsc + SC_CURSOR))[1];
-  if (dev_err & ERR_FRONTIER_FULL) { set_err(c, "frontier capacity %llu exceeded", (unsigned long long)c->fr.cap); return TGI_E_CAPACITY; }
-  if (dev_err & 16) { set_err(c, "internal: sized and emitted line lengths disagree"); return TGI_E_STATE; }
-  n_links_total = want_links ? hsc[SC_LINK_TOTAL] : 0;
+  const int rc = device_errors(c, ((int*)(hsc + SC_CURSOR))[1]);
+  if (rc) return rc;
+  const uint64_t n_links_total = want_links ? hsc[SC_LINK_TOTAL] : 0;
   if (n_links_total > arena_used) { set_err(c, "internal: more links than arena rows"); return TGI_E_STATE; }
-  float ms = 0;
-  cudaEventElapsedTime(&ms, s.ev_k0, s.ev_k1);
-  out->kernel_ms = ms;
-  out->gpu_launches = launches;
-  out->slot = s.idx;
+  fill_result(c, s, n, flags, hsc, line_total, n_links_total, launches, out);
   if (n) cudaEventElapsedTime(&out->parse_ms, s.ev_p0, s.ev_p1);
   if (n && want_json) {
     cudaEventElapsedTime(&out->emit_ms, s.ev_e0, s.ev_e1);
     cudaEventElapsedTime(&out->emit_main_ms, s.ev_e0, s.ev_f1);
-    out->var_bytes = var_bytes;
-    out->main_bytes_out = hsc[SC_LANE_OUT];
-    out->main_bytes_in = hsc[SC_LANE_IN];
   }
   if (want_fr && n) cudaEventElapsedTime(&out->frontier_ms, s.ev_fr0, s.ev_fr1);
-  out->jsonl_len = want_json ? line_total : 0;
-  out->n_links = n_links_total;
-  out->n_new = want_fr ? hsc[SC_NEW] : 0;
-  s.last_n = n;
-  s.last_new = out->n_new;
-  s.last_frontier = want_fr && n;
-  s.last_yt = s.tg.n == 0 && s.yt.n == n && n != 0;
-  out->frontier_size = want_fr ? hsc[SC_FSIZE] : 0;
   if (d2h) {
     out->status = s.h_status.as<uint8_t>();
     if (want_json) {
@@ -740,27 +739,12 @@ int finish_batch(tgi_ctx* c, Slot& s, uint64_t n, uint32_t flags, uint64_t line_
       out->links = s.h_links.as<tgi_link>();
     }
   }
-  {
-    std::lock_guard<std::mutex> g(c->st_mu);
-    c->stats.records += n;
-    c->stats.bytes_in += s.in_bytes;
-    c->stats.bytes_out += out->jsonl_len;
-    c->stats.links += n_links_total;
-    c->stats.launches += launches;
-    c->stats.kernel_ms_total += ms;
-    if (want_fr) c->stats.frontier_size = out->frontier_size;
-  }
   return TGI_OK;
 }
 
 // One cooperative launch and one result copy for a page-sized batch.  PAGE_FALLBACK: the batch did not fit the
-// estimate-sized result block or the link arena (nothing was committed): run_tg goes on with the ordinary pipeline.
+// estimate-sized result block or the link arena (nothing was committed): the caller goes on with the ordinary pipeline.
 constexpr int PAGE_FALLBACK = -1000;
-bool page_run_ok(const Slot& s, uint32_t flags) {
-  if (!page_enabled() || s.tg.n == 0 || s.tg.n > PAGE_MAX_RECS || s.tg.n_chans > PAGE_MAX_RECS || s.in_bytes > PAGE_MAX_IN_BYTES) return false;
-  if (flags & TGI_RUN_NO_D2H) return false;  // a device-resident result keeps the ordinary buffers
-  return (flags & (TGI_RUN_JSONL | TGI_RUN_LINKS | TGI_RUN_FRONTIER)) != 0;
-}
 // ---- shared by the Telegram and the YouTube page paths ------------------------------------------------------------------
 struct PageOut {  // the result block: scalars | status | line_off | link_off | links, JSONL
   uint64_t o_status, o_line_off, o_link_off, o_var, var_cap;
@@ -779,7 +763,7 @@ int page_out_prepare(tgi_ctx* c, Slot& s, uint64_t n, PageOut& L) {
 }
 // launch (in the batch's frontier turn), ONE read of the result block, the result.  PAGE_FALLBACK: nothing was committed.
 int page_launch_and_read(tgi_ctx* c, Slot& s, uint32_t flags, uint64_t n, const void* kernel, void** kargs, int occ, const PageOut& L,
-                         FrontierDev* fr_arg, ExclusionDev* excl_arg, const char* name, bool is_yt, tgi_result* out) {
+                         FrontierDev* fr_arg, ExclusionDev* excl_arg, const char* name, tgi_result* out) {
   cudaStream_t st = s.stream;
   const bool want_json = flags & TGI_RUN_JSONL, want_links = flags & TGI_RUN_LINKS, want_fr = flags & TGI_RUN_FRONTIER;
   auto up = [](uint64_t v, uint64_t a) { return (v + a - 1) / a * a; };
@@ -816,13 +800,13 @@ int page_launch_and_read(tgi_ctx* c, Slot& s, uint32_t flags, uint64_t n, const 
   const int dev_err = ((const int*)(hsc + SC_CURSOR))[1];
   if (dev_err & (ERR_ARENA_OVERFLOW | ERR_TOO_MANY_LINKS | ERR_PAGE_OVERFLOW)) return PAGE_FALLBACK;  // keeps its turn
   turn_end(c, s);
-  if (dev_err & ERR_FRONTIER_FULL) { set_err(c, "frontier capacity %llu exceeded", (unsigned long long)c->fr.cap); return TGI_E_CAPACITY; }
-  if (dev_err & 16) { set_err(c, "internal: sized and emitted line lengths disagree"); return TGI_E_STATE; }
+  int rc = device_errors(c, dev_err);
+  if (rc) return rc;
   const uint64_t line_total = want_json ? hsc[SC_LINE_TOTAL] : 0, n_links_total = want_links ? hsc[SC_LINK_TOTAL] : 0;
   const uint64_t links_bytes = want_links ? up(n_links_total * sizeof(tgi_link), 256) : 0;
-  if (want_json && c->cfg.max_out_bytes && line_total > c->cfg.max_out_bytes) {
-    set_err(c, "JSONL output %llu bytes exceeds max_out_bytes", (unsigned long long)line_total);
-    return TGI_E_CAPACITY;
+  if (want_json) {
+    rc = check_out_bytes(c, line_total);
+    if (rc) return rc;
   }
   const uint64_t need = links_bytes + line_total;
   if (need > spec) {
@@ -842,21 +826,7 @@ int page_launch_and_read(tgi_ctx* c, Slot& s, uint32_t flags, uint64_t n, const 
   s.page_bpr = (uint32_t)std::min<uint64_t>(1u << 20, (3ull * s.page_bpr + need / n + 1) / 4 + (need > spec ? need / n / 4 : 0));
 
   memset(out, 0, sizeof *out);
-  out->n = n;
-  float ms = 0;
-  cudaEventElapsedTime(&ms, s.ev_k0, s.ev_k1);
-  out->kernel_ms = ms;
-  out->gpu_launches = 1;
-  out->slot = s.idx;
-  if (want_json) {
-    out->var_bytes = hsc[SC_LONG];
-    out->main_bytes_out = hsc[SC_LANE_OUT];
-    out->main_bytes_in = hsc[SC_LANE_IN];
-  }
-  out->jsonl_len = line_total;
-  out->n_links = n_links_total;
-  out->n_new = want_fr ? hsc[SC_NEW] : 0;
-  out->frontier_size = want_fr ? hsc[SC_FSIZE] : 0;
+  fill_result(c, s, n, flags, hsc, line_total, n_links_total, 1, out);
   out->status = h + o_status;
   if (want_json) {
     out->jsonl = h + o_var + links_bytes;
@@ -868,28 +838,13 @@ int page_launch_and_read(tgi_ctx* c, Slot& s, uint32_t flags, uint64_t n, const 
   }
   s.dev_jsonl_len = line_total;
   s.dev_jsonl = d + o_var + links_bytes;
-  s.last_n = n;
-  s.last_new = out->n_new;
-  s.last_frontier = want_fr;
-  s.last_yt = is_yt;
-  {
-    std::lock_guard<std::mutex> g(c->st_mu);
-    c->stats.records += n;
-    c->stats.bytes_in += s.in_bytes;
-    c->stats.bytes_out += out->jsonl_len;
-    c->stats.links += n_links_total;
-    c->stats.launches += 1;
-    c->stats.kernel_ms_total += ms;
-    if (want_fr) c->stats.frontier_size = out->frontier_size;
-  }
   return TGI_OK;
 }
 
 
-int run_tg_page(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
+int run_tg_page(tgi_ctx* c, Slot& s, const CfgDev& cfg, uint32_t flags, tgi_result* out) {
   TgBatchDev& b = s.tg;
   const uint64_t n = b.n;
-  const bool want_fr = flags & TGI_RUN_FRONTIER;
   static const int occ = [] {
     int o = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, tg_page_kernel, CTA_THREADS, 0) != cudaSuccess) return 0;
@@ -897,14 +852,10 @@ int run_tg_page(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
   }();
   if (occ <= 0) { cudaGetLastError(); return PAGE_FALLBACK; }
   PageArgs pa{};
-  {
-    std::lock_guard<std::mutex> g(c->cfg_mu);
-    pa.cfg = c->cfgdev;
-  }
+  pa.cfg = cfg;
   pa.run_flags = flags;
   const uint64_t arena_cap = s.n_ents + 2 * n + 1024;
   const uint64_t blob_cap = 8 * s.chan_strs_len + 1024ull * b.n_chans + 1024;
-  const uint64_t bslots = next_pow2(std::max<uint64_t>(2 * arena_cap, 1024));
   // scratch (the buffers of the ordinary pipeline, so that tgi_pending_edges finds the same arrays afterwards)
   CK(s.d_linelen.ensure(n * 4));
   CK(s.d_link_start.ensure(n * 4));
@@ -919,11 +870,9 @@ int run_tg_page(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
   CK(s.d_chan_len.ensure((size_t)b.n_chans * 4));
   CK(s.d_chan_off.ensure(((size_t)b.n_chans + 1) * 8));
   CK(s.d_chan_blob.ensure(blob_cap));
-  if (want_fr) {
-    CK(s.d_btable.ensure(bslots * 8));
-    CK(s.d_lstate.ensure((size_t)arena_cap * 4));
-    CK(s.d_rec_new.ensure(n * 4));
-    CK(s.d_new_off.ensure((n + 1) * 8));
+  if (flags & TGI_RUN_FRONTIER) {
+    const int rc = frontier_scratch(c, s, n, arena_cap, arena_cap, pa.fb);
+    if (rc) return rc;
   }
   PageOut L;
   {
@@ -976,36 +925,22 @@ int run_tg_page(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
   pa.var_cap = var_cap;
   pa.max_out = c->cfg.max_out_bytes;
   pa.fr = c->fr;
-  pa.fb.btable = s.d_btable.as<uint64_t>();
-  pa.fb.bmask = bslots - 1;
-  pa.fb.lstate = s.d_lstate.as<uint32_t>();
-  pa.fb.rec_new = s.d_rec_new.as<uint32_t>();
   pa.excl = c->excl;
-  pa.bslots = bslots;
+  pa.bslots = pa.fb.bmask + 1;
   pa.new_off = s.d_new_off.as<uint64_t>();
-  pa.sc_chan_total = SC_CHAN_TOTAL;
-  pa.sc_line_total = SC_LINE_TOTAL;
-  pa.sc_link_total = SC_LINK_TOTAL;
-  pa.sc_new = SC_NEW;
-  pa.sc_count = SC_COUNT;
 
   void* kargs[] = {&pa};
-  return page_launch_and_read(c, s, flags, n, (const void*)tg_page_kernel, kargs, occ, L, &pa.fr, &pa.excl, "tg_page", false, out);
+  return page_launch_and_read(c, s, flags, n, (const void*)tg_page_kernel, kargs, occ, L, &pa.fr, &pa.excl, "tg_page", out);
 }
 
-int run_tg(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
+int run_tg(tgi_ctx* c, Slot& s, const CfgDev& cfg, uint32_t flags, tgi_result* out) {
   TgBatchDev& b = s.tg;
   uint64_t n = b.n;
   cudaStream_t st = s.stream;
   uint32_t launches = 0;
   const bool want_json = flags & TGI_RUN_JSONL;
-  CfgDev cfg;
-  {
-    std::lock_guard<std::mutex> g(c->cfg_mu);
-    cfg = c->cfgdev;
-  }
-  if (page_run_ok(s, flags)) {
-    const int rc = run_tg_page(c, s, flags, out);
+  if (page_run(s, n, b.n_chans, flags)) {
+    const int rc = run_tg_page(c, s, cfg, flags, out);
     if (rc != PAGE_FALLBACK) return rc;
   }
   CK(s.d_scalars.ensure(SC_COUNT * 8));
@@ -1096,13 +1031,10 @@ int run_tg(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
   if (dev_err & ERR_TOO_MANY_LINKS) { set_err(c, "a record has 2^20 or more link candidates"); return TGI_E_ARG; }
   uint64_t chan_total = hsc[SC_CHAN_TOTAL], line_total = hsc[SC_LINE_TOTAL];
   uint32_t arena_used = ((uint32_t*)(hsc + SC_CURSOR))[0];
-  const uint64_t var_bytes = hsc[SC_LONG];
 
   if (want_json) {
-    if (c->cfg.max_out_bytes && line_total > c->cfg.max_out_bytes) {
-      set_err(c, "JSONL output %llu bytes exceeds max_out_bytes", (unsigned long long)line_total);
-      return TGI_E_CAPACITY;
-    }
+    const int rc = check_out_bytes(c, line_total);
+    if (rc) return rc;
     CK(s.d_chan_blob.ensure(chan_total));
     CK(s.d_jsonl.ensure(line_total));
     if (chan_total) CK(cudaMemsetAsync(s.d_chan_blob.p, 0, chan_total, st));  // segment padding must read as zero
@@ -1142,22 +1074,15 @@ int run_tg(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
       tg_emit_lane_kernel<<<gl, CTA_THREADS, sizeof(LaneShared), st>>>(b, cfg, ei);
       CK(cudaEventRecord(s.ev_f1, st));
       unsigned gg = (unsigned)std::min<uint64_t>(ctas, (uint64_t)c->sms * grid_mult());
-      static const bool one_esc = getenv("TGI_ESC_ONE") != nullptr;  // A/B: the round-1 single escape kernel
-      if (one_esc) {
-        tg_emit_esc_kernel<ESC_ALL><<<gg, CTA_THREADS, 0, st>>>(b, ei);
-        launches += 1;
-      } else {
-        tg_emit_esc_kernel<ESC_SPARSE><<<gg, CTA_THREADS, 0, st>>>(b, ei);  // descriptions with a few line breaks
-        tg_emit_esc_kernel<ESC_DENSE><<<gg, CTA_THREADS, 0, st>>>(b, ei);   // the other strings that need escaping or are long
-        launches += 2;
-      }
+      tg_emit_esc_kernel<ESC_SPARSE><<<gg, CTA_THREADS, 0, st>>>(b, ei);  // descriptions with a few line breaks
+      tg_emit_esc_kernel<ESC_DENSE><<<gg, CTA_THREADS, 0, st>>>(b, ei);   // the other strings that need escaping or are long
       tg_emit_maps_kernel<<<gg, CTA_THREADS, 0, st>>>(b, ei);  // comment lists, non-trivial maps, long outlink lists
-      launches += 2;
+      launches += 4;
       CK(cudaEventRecord(s.ev_e1, st));
     }
     CK(cudaGetLastError());
   }
-  return finish_batch(c, s, n, flags, line_total, arena_used, arena_cap, var_bytes, launches, out);
+  return finish_batch(c, s, n, flags, line_total, arena_used, arena_cap, launches, out);
 }
 
 int upload_yt(tgi_ctx* c, Slot& s, const tgi_yt_batch* in) {
@@ -1179,56 +1104,31 @@ int upload_yt(tgi_ctx* c, Slot& s, const tgi_yt_batch* in) {
     }
     if (e) { set_err(c, "youtube batch: offsets outside their arrays (mask 0x%x)", e); return TGI_E_ARG; }
   }
-  s.in_bytes = 0;
-  int rc;
-  YtBatchDev& b = s.yt;
-  const size_t yb[4] = {in->n * sizeof(tgi_yt_rec), in->strs_len, in->n_chans * sizeof(tgi_yt_chan), in->chan_strs_len};
-  size_t yo[5] = {0, 0, 0, 0, 0};
-  for (int i = 0; i < 4; i++) yo[i + 1] = yo[i] + ((yb[i] + PAD + 15) & ~(size_t)15);
-  if (page_enabled() && in->n && in->n <= PAGE_MAX_RECS && in->n_chans <= PAGE_MAX_RECS && yo[4] <= PAGE_MAX_IN_BYTES) {
-    // page-sized: the four arrays in one pinned block, ONE copy (upload_tg_page)
-    CK(s.h_page_in.ensure(yo[4]));
-    CK(s.d_page_in.ensure(yo[4]));
-    uint8_t* h = s.h_page_in.as<uint8_t>();
-    const void* src[4] = {in->recs, in->strs, in->chans, in->chan_strs};
-    for (int i = 0; i < 4; i++) {
-      if (yb[i]) memcpy(h + yo[i], src[i], yb[i]);
-      memset(h + yo[i] + yb[i], 0, yo[i + 1] - yo[i] - yb[i]);
-      s.in_bytes += yb[i];
-    }
-    CK(cudaMemcpyAsync(s.d_page_in.p, h, yo[4], cudaMemcpyHostToDevice, s.stream));
-    uint8_t* d = s.d_page_in.as<uint8_t>();
-    b.recs = (const tgi_yt_rec*)(d + yo[0]);
-    b.strs = d + yo[1];
-    b.chans = (const tgi_yt_chan*)(d + yo[2]);
-    b.chan_strs = d + yo[3];
-  } else {
-#define UP(buf, ptr, cnt)                      \
-  rc = h2d(c, s, s.buf, ptr, (size_t)(cnt));   \
+  const InArray arr[4] = {{&s.d_recs, in->recs, in->n * sizeof(tgi_yt_rec)},
+                          {&s.d_strs, in->strs, in->strs_len},
+                          {&s.d_chans, in->chans, in->n_chans * sizeof(tgi_yt_chan)},
+                          {&s.d_chan_strs, in->chan_strs, in->chan_strs_len}};
+  const uint8_t* d[4];
+  const int rc = upload_arrays(c, s, arr, 4, page_sized(in->n, in->n_chans, packed_size(arr, 4)), d);
   if (rc) return rc;
-    UP(d_recs, in->recs, in->n);
-    UP(d_strs, in->strs, in->strs_len);
-    UP(d_chans, in->chans, in->n_chans);
-    UP(d_chan_strs, in->chan_strs, in->chan_strs_len);
-#undef UP
-    b.recs = s.d_recs.as<tgi_yt_rec>();
-    b.strs = s.d_strs.as<uint8_t>();
-    b.chans = s.d_chans.as<tgi_yt_chan>();
-    b.chan_strs = s.d_chan_strs.as<uint8_t>();
-  }
+  YtBatchDev& b = s.yt;
   b.n = in->n;
+  b.recs = (const tgi_yt_rec*)d[0];
+  b.strs = d[1];
   b.n_chans = in->n_chans;
+  b.chans = (const tgi_yt_chan*)d[2];
+  b.chan_strs = d[3];
   s.yt_desc_bytes = in->strs_len;
+  s.batch = JOB_YT;
   s.resident = true;
-  s.tg.n = 0;
+  s.tg.n = 0;  // the slot no longer holds a Telegram batch: a Telegram resident run finds an empty one
   return TGI_OK;
 }
 
 // a page of the Data API (50 videos) in one cooperative launch (yt_page.cuh); PAGE_FALLBACK as in run_tg_page
-int run_yt_page(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
+int run_yt_page(tgi_ctx* c, Slot& s, const CfgDev& cfg, uint32_t flags, tgi_result* out) {
   YtBatchDev& b = s.yt;
   const uint64_t n = b.n;
-  const bool want_fr = flags & TGI_RUN_FRONTIER;
   static const int occ = [] {
     int o = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, yt_page_kernel, CTA_THREADS, 0) != cudaSuccess) return 0;
@@ -1236,15 +1136,11 @@ int run_yt_page(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
   }();
   if (occ <= 0) { cudaGetLastError(); return PAGE_FALLBACK; }
   YtPageArgs pa{};
-  {
-    std::lock_guard<std::mutex> g(c->cfg_mu);
-    pa.cfg = c->cfgdev;
-  }
+  pa.cfg = cfg;
   pa.run_flags = flags;
   pa.b = b;
   // every URL needs "http://x" (8 bytes), every channel link "youtube.com/" (12 bytes): upper bounds, as in run_yt
   const uint64_t urls_cap = s.yt_desc_bytes / 4 + 1024, arena_cap = s.yt_desc_bytes / 12 + 1024;
-  const uint64_t bslots = next_pow2(std::max<uint64_t>(2 * arena_cap, 1024));
   CK(s.d_linelen.ensure(n * 4));
   CK(s.d_link_start.ensure(n * 4));
   CK(s.d_link_count.ensure(n * 4));
@@ -1254,11 +1150,9 @@ int run_yt_page(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
   CK(s.d_arena.ensure(arena_cap * sizeof(tgi_link)));
   CK(s.d_xlen.ensure(n * 12));
   CK(s.d_link_off.ensure((n + 1) * 8));
-  if (want_fr) {
-    CK(s.d_btable.ensure(bslots * 8));
-    CK(s.d_lstate.ensure((size_t)arena_cap * 4));
-    CK(s.d_rec_new.ensure(n * 4));
-    CK(s.d_new_off.ensure((n + 1) * 8));
+  if (flags & TGI_RUN_FRONTIER) {
+    const int rc = frontier_scratch(c, s, n, arena_cap, arena_cap, pa.fb);
+    if (rc) return rc;
   }
   PageOut L;
   {
@@ -1290,36 +1184,22 @@ int run_yt_page(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
   pa.var_cap = L.var_cap;
   pa.max_out = c->cfg.max_out_bytes;
   pa.fr = c->fr;
-  pa.fb.btable = s.d_btable.as<uint64_t>();
-  pa.fb.bmask = bslots - 1;
-  pa.fb.lstate = s.d_lstate.as<uint32_t>();
-  pa.fb.rec_new = s.d_rec_new.as<uint32_t>();
   pa.excl = c->excl;
-  pa.bslots = bslots;
+  pa.bslots = pa.fb.bmask + 1;
   pa.new_off = s.d_new_off.as<uint64_t>();
-  pa.sc_line_total = SC_LINE_TOTAL;
-  pa.sc_link_total = SC_LINK_TOTAL;
-  pa.sc_new = SC_NEW;
-  pa.sc_count = SC_COUNT;
   void* kargs[] = {&pa};
-  return page_launch_and_read(c, s, flags, n, (const void*)yt_page_kernel, kargs, occ, L, &pa.fr, &pa.excl, "yt_page", true, out);
+  return page_launch_and_read(c, s, flags, n, (const void*)yt_page_kernel, kargs, occ, L, &pa.fr, &pa.excl, "yt_page", out);
 }
 
-int run_yt(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
+int run_yt(tgi_ctx* c, Slot& s, const CfgDev& cfg, uint32_t flags, tgi_result* out) {
   YtBatchDev& b = s.yt;
   uint64_t n = b.n;
   cudaStream_t st = s.stream;
   uint32_t launches = 0;
   const bool want_json = flags & TGI_RUN_JSONL;
-  if (page_enabled() && n && n <= PAGE_MAX_RECS && b.n_chans <= PAGE_MAX_RECS && s.in_bytes <= PAGE_MAX_IN_BYTES && !(flags & TGI_RUN_NO_D2H) &&
-      (flags & (TGI_RUN_JSONL | TGI_RUN_LINKS | TGI_RUN_FRONTIER))) {
-    const int rc = run_yt_page(c, s, flags, out);
+  if (page_run(s, n, b.n_chans, flags)) {
+    const int rc = run_yt_page(c, s, cfg, flags, out);
     if (rc != PAGE_FALLBACK) return rc;
-  }
-  CfgDev cfg;
-  {
-    std::lock_guard<std::mutex> g(c->cfg_mu);
-    cfg = c->cfgdev;
   }
   CK(s.d_scalars.ensure(SC_COUNT * 8));
   CK(s.h_scalars.ensure(SC_COUNT * 8));
@@ -1355,19 +1235,14 @@ int run_yt(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
   yo.cursor = (uint32_t*)(dsc + SC_CURSOR);
   yo.err = (int*)(dsc + SC_CURSOR) + 1;
   unsigned g = (unsigned)std::min<uint64_t>((n + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (uint64_t)c->sms * grid_mult());
+  // the lane kernels: one warp per 32 records
+  unsigned gl = (unsigned)std::min<uint64_t>(((n + 31) / 32 + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (uint64_t)c->sms * grid_mult());
   if (n) {
     CK(cudaEventRecord(s.ev_p0, st));
     yt_parse_kernel<<<g, CTA_THREADS, 0, st>>>(b, cfg, flags, yo);
     launches++;
     if (want_json) {
-      static const bool yt_warp = getenv("TGI_YT_WARP") != nullptr;
-      if (yt_warp) {
-        yt_size_kernel<<<g, CTA_THREADS, 0, st>>>(b, cfg, yo);
-      } else {
-        const uint64_t groups = (n + 31) / 32;
-        unsigned gs = (unsigned)std::min<uint64_t>((groups + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (uint64_t)c->sms * grid_mult());
-        yt_size_lane_kernel<<<gs, CTA_THREADS, 0, st>>>(b, cfg, yo);
-      }
+      yt_size_lane_kernel<<<gl, CTA_THREADS, 0, st>>>(b, cfg, yo);
       launches++;
     }
     CK(cudaEventRecord(s.ev_p1, st));
@@ -1389,32 +1264,25 @@ int run_yt(tgi_ctx* c, Slot& s, uint32_t flags, tgi_result* out) {
   uint64_t line_total = hsc[SC_LINE_TOTAL];
   uint32_t arena_used = ((uint32_t*)(hsc + SC_CURSOR))[0];
   if (want_json) {
-    if (c->cfg.max_out_bytes && line_total > c->cfg.max_out_bytes) {
-      set_err(c, "JSONL output %llu bytes exceeds max_out_bytes", (unsigned long long)line_total);
-      return TGI_E_CAPACITY;
-    }
+    const int rc = check_out_bytes(c, line_total);
+    if (rc) return rc;
     CK(s.d_jsonl.ensure(line_total));
     if (n) {
       CK(cudaEventRecord(s.ev_e0, st));
-      static const bool yt_warp = getenv("TGI_YT_WARP") != nullptr;  // A/B switch: the warp writer for every record
-      const uint64_t groups = (n + 31) / 32;
-      unsigned gg = (unsigned)std::min<uint64_t>((groups + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (uint64_t)c->sms * grid_mult());
-      if (!yt_warp) {
-        yt_emit_lane_kernel<<<gg, CTA_THREADS, 0, st>>>(b, cfg, yo, s.d_line_off.as<uint64_t>(), s.d_jsonl.as<uint8_t>(), yo.err);
-        launches++;
-      }
-      yt_emit_kernel<<<gg, CTA_THREADS, 0, st>>>(b, cfg, yo, s.d_line_off.as<uint64_t>(), s.d_jsonl.as<uint8_t>(), yo.err, yt_warp ? 0 : 1);
+      // the lane writer takes the clean records, the warp writer the ones with a string that needs escaping
+      yt_emit_lane_kernel<<<gl, CTA_THREADS, 0, st>>>(b, cfg, yo, s.d_line_off.as<uint64_t>(), s.d_jsonl.as<uint8_t>(), yo.err);
+      yt_emit_kernel<<<gl, CTA_THREADS, 0, st>>>(b, cfg, yo, s.d_line_off.as<uint64_t>(), s.d_jsonl.as<uint8_t>(), yo.err);
       CK(cudaEventRecord(s.ev_f1, st));
       CK(cudaEventRecord(s.ev_e1, st));
-      launches++;
+      launches += 2;
     }
     CK(cudaGetLastError());
   }
-  return finish_batch(c, s, n, flags, line_total, arena_used, arena_cap, 0, launches, out);
+  return finish_batch(c, s, n, flags, line_total, arena_used, arena_cap, launches, out);
 }
 
 // generic client.Message batch (a12): upload, size, scan, emit; no links
-int run_gm(tgi_ctx* c, Slot& s, const tgi_gm_batch* in, uint32_t flags, tgi_result* out) {
+int run_gm(tgi_ctx* c, Slot& s, const CfgDev& cfg, const tgi_gm_batch* in, uint32_t flags, tgi_result* out) {
   if (!in) { set_err(c, "null batch"); return TGI_E_ARG; }
   if (in->n && !in->recs) { set_err(c, "generic batch: recs must be non-null"); return TGI_E_ARG; }
   if (in->n >= (1ull << 40)) { set_err(c, "generic batch: too many records"); return TGI_E_ARG; }
@@ -1432,32 +1300,25 @@ int run_gm(tgi_ctx* c, Slot& s, const tgi_gm_batch* in, uint32_t flags, tgi_resu
   }
   const uint64_t n = in->n;
   cudaStream_t st = s.stream;
-  s.in_bytes = 0;
   s.resident = false;
-  int rc;
-#define UP(buf, ptr, cnt)                      \
-  rc = h2d(c, s, s.buf, ptr, (size_t)(cnt));   \
+  const InArray arr[5] = {{&s.d_recs, in->recs, n * sizeof(tgi_gm_rec)},
+                          {&s.d_strs, in->strs, in->strs_len},
+                          {&s.d_react_off, in->react_off, in->react_off ? (n + 1) * 4 : 0},
+                          {&s.d_reacts, in->reacts, in->n_reacts * sizeof(tgi_gm_reaction)},
+                          {&s.d_aux, in->aux, in->aux_len}};
+  const uint8_t* d[5];
+  int rc = upload_arrays(c, s, arr, 5, false, d);
   if (rc) return rc;
-  UP(d_recs, in->recs, n);
-  UP(d_strs, in->strs, in->strs_len);
-  UP(d_react_off, in->react_off, in->react_off ? n + 1 : 0);
-  UP(d_reacts, in->reacts, in->n_reacts);
-  UP(d_aux, in->aux, in->aux_len);
-#undef UP
   GmBatchDev& b = s.gm;
   b.n = n;
-  b.recs = s.d_recs.as<tgi_gm_rec>();
-  b.strs = s.d_strs.as<uint8_t>();
-  b.react_off = in->react_off ? s.d_react_off.as<uint32_t>() : nullptr;
-  b.reacts = s.d_reacts.as<tgi_gm_reaction>();
-  b.aux = s.d_aux.as<uint8_t>();
+  b.recs = (const tgi_gm_rec*)d[0];
+  b.strs = d[1];
+  b.react_off = in->react_off ? (const uint32_t*)d[2] : nullptr;
+  b.reacts = (const tgi_gm_reaction*)d[3];
+  b.aux = d[4];
+  s.batch = JOB_GM;
   uint32_t launches = 0;
   const bool want_json = flags & TGI_RUN_JSONL;
-  CfgDev cfg;
-  {
-    std::lock_guard<std::mutex> g(c->cfg_mu);
-    cfg = c->cfgdev;
-  }
   CK(s.d_scalars.ensure(SC_COUNT * 8));
   CK(s.h_scalars.ensure(SC_COUNT * 8));
   uint64_t* dsc = s.d_scalars.as<uint64_t>();
@@ -1491,10 +1352,8 @@ int run_gm(tgi_ctx* c, Slot& s, const tgi_gm_batch* in, uint32_t flags, tgi_resu
     launches++;
     CK(cudaStreamSynchronize(st));
     line_total = hsc[SC_LINE_TOTAL];
-    if (c->cfg.max_out_bytes && line_total > c->cfg.max_out_bytes) {
-      set_err(c, "JSONL output %llu bytes exceeds max_out_bytes", (unsigned long long)line_total);
-      return TGI_E_CAPACITY;
-    }
+    rc = check_out_bytes(c, line_total);
+    if (rc) return rc;
     CK(s.d_jsonl.ensure(line_total));
     CK(cudaEventRecord(s.ev_e0, st));
     if (n) {
@@ -1505,7 +1364,29 @@ int run_gm(tgi_ctx* c, Slot& s, const tgi_gm_batch* in, uint32_t flags, tgi_resu
     CK(cudaEventRecord(s.ev_e1, st));
     CK(cudaGetLastError());
   }
-  return finish_batch(c, s, n, flags & ~(uint32_t)TGI_RUN_FRONTIER, line_total, 0, 1024, 0, launches, out);
+  return finish_batch(c, s, n, flags & ~(uint32_t)TGI_RUN_FRONTIER, line_total, 0, 1024, launches, out);
+}
+
+// One job on the slot, with the inputs and flags the slot holds: upload (JOB_TG, JOB_YT, the *_UPLOAD kinds), run
+// (JOB_TG, JOB_YT, the *_RESIDENT kinds, JOB_GM), then the job's frontier turn if the run did not take it.
+int run_job(tgi_ctx* c, Slot& s, JobKind kind) {
+  CfgDev cfg;
+  {
+    std::lock_guard<std::mutex> g(c->cfg_mu);
+    cfg = c->cfgdev;
+  }
+  int rc = TGI_OK;
+  if (kind == JOB_TG || kind == JOB_TG_UPLOAD) rc = upload_tg(c, s, s.in_tg);
+  if (kind == JOB_YT || kind == JOB_YT_UPLOAD) rc = upload_yt(c, s, s.in_yt);
+  if (rc == TGI_OK && (kind == JOB_TG_UPLOAD || kind == JOB_YT_UPLOAD)) {
+    const cudaError_t e = cudaStreamSynchronize(s.stream);
+    if (e != cudaSuccess) { set_err(c, "upload sync: %s", cudaGetErrorString(e)); rc = TGI_E_CUDA; }
+  }
+  if (rc == TGI_OK && (kind == JOB_TG || kind == JOB_TG_RESIDENT)) rc = run_tg(c, s, cfg, s.run_flags, &s.res);
+  if (rc == TGI_OK && (kind == JOB_YT || kind == JOB_YT_RESIDENT)) rc = run_yt(c, s, cfg, s.run_flags, &s.res);
+  if (kind == JOB_GM) rc = run_gm(c, s, cfg, s.in_gm, s.run_flags, &s.res);
+  turn_pass(c, s);
+  return rc;
 }
 
 void worker_main(tgi_ctx* c, Slot* s) {
@@ -1518,21 +1399,7 @@ void worker_main(tgi_ctx* c, Slot* s) {
       job = s->job;
     }
     if (job == JOB_QUIT) return;
-    int rc = TGI_OK;
-    if (job == JOB_TG || job == JOB_TG_UPLOAD) rc = upload_tg(c, *s, s->in_tg);
-    if (rc == TGI_OK && job == JOB_TG_UPLOAD) {
-      cudaError_t e = cudaStreamSynchronize(s->stream);
-      if (e != cudaSuccess) { set_err(c, "upload sync: %s", cudaGetErrorString(e)); rc = TGI_E_CUDA; }
-    }
-    if (rc == TGI_OK && (job == JOB_TG || job == JOB_TG_RESIDENT)) rc = run_tg(c, *s, s->run_flags, &s->res);
-    if (job == JOB_YT || job == JOB_YT_UPLOAD) rc = upload_yt(c, *s, s->in_yt);
-    if (rc == TGI_OK && job == JOB_YT_UPLOAD) {
-      cudaError_t e = cudaStreamSynchronize(s->stream);
-      if (e != cudaSuccess) { set_err(c, "upload sync: %s", cudaGetErrorString(e)); rc = TGI_E_CUDA; }
-    }
-    if (rc == TGI_OK && (job == JOB_YT || job == JOB_YT_RESIDENT)) rc = run_yt(c, *s, s->run_flags, &s->res);
-    if (job == JOB_GM) rc = run_gm(c, *s, s->in_gm, s->run_flags, &s->res);
-    turn_pass(c, *s);
+    const int rc = run_job(c, *s, job);
     {
       std::lock_guard<std::mutex> lk(s->mu);
       s->rc = rc;
@@ -1586,20 +1453,14 @@ int run_inline(tgi_ctx* c, int slot, JobKind kind, const tgi_tg_batch* in_tg, co
     if (s.busy) { set_err(c, "slot %d is busy", slot); return TGI_E_STATE; }
     s.busy = true;
     s.done = false;
+    s.in_tg = in_tg;
+    s.in_yt = in_yt;
+    s.in_gm = in_gm;
+    s.run_flags = flags;
   }
   take_ticket(c, s, kind, flags);
   cudaSetDevice(c->device);
-  int rc = TGI_OK;
-  if (kind == JOB_TG) {
-    rc = upload_tg(c, s, in_tg);
-    if (rc == TGI_OK) rc = run_tg(c, s, flags, &s.res);
-  } else if (kind == JOB_YT) {
-    rc = upload_yt(c, s, in_yt);
-    if (rc == TGI_OK) rc = run_yt(c, s, flags, &s.res);
-  } else {
-    rc = run_gm(c, s, in_gm, flags, &s.res);
-  }
-  turn_pass(c, s);
+  const int rc = run_job(c, s, kind);
   {
     std::lock_guard<std::mutex> lk(s.mu);
     s.rc = rc;
@@ -2197,8 +2058,9 @@ int tgi_pending_edges(tgi_ctx* c, int slot, int64_t now_sec, tgi_edge* rows, uin
   ExclusionDev x = c->excl;
   x.now_sec = now_sec;
   // the resident batch descriptor, not the upload buffers: a page-sized batch lives in the slot's one-block upload
-  const uint32_t* chan = s.last_yt ? &s.yt.recs->chan_idx : &s.tg.recs->chan_idx;
-  const uint32_t stride = s.last_yt ? (uint32_t)sizeof(tgi_yt_rec) : (uint32_t)sizeof(tgi_tg_rec);
+  const bool yt = s.batch == JOB_YT;
+  const uint32_t* chan = yt ? &s.yt.recs->chan_idx : &s.tg.recs->chan_idx;
+  const uint32_t stride = yt ? (uint32_t)sizeof(tgi_yt_rec) : (uint32_t)sizeof(tgi_tg_rec);
   edges_emit_kernel<<<(unsigned)((s.last_n + 255) / 256), 256, 0, st>>>(s.last_n, s.d_link_start.as<uint32_t>(), s.d_link_count.as<uint32_t>(),
                                                                     s.d_arena.as<tgi_link>(), chan, stride, s.d_new_off.as<uint64_t>(), x,
                                                                     drows.as<tgi_edge>(), m);

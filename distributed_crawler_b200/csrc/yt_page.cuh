@@ -32,7 +32,6 @@ struct YtPageArgs {
   ExclusionDev excl;
   uint64_t bslots;
   uint64_t* new_off;
-  int sc_line_total, sc_link_total, sc_new, sc_count;
 };
 
 __global__ void __launch_bounds__(CTA_THREADS, 2) yt_page_kernel(const __grid_constant__ YtPageArgs a) {
@@ -56,7 +55,7 @@ __global__ void __launch_bounds__(CTA_THREADS, 2) yt_page_kernel(const __grid_co
   stamp();
 
   // P0
-  if (blockIdx.x == 0 && (int)threadIdx.x < a.sc_count) a.scalars[threadIdx.x] = 0;
+  if (blockIdx.x == 0 && threadIdx.x < SC_COUNT) a.scalars[threadIdx.x] = 0;
   if (blockIdx.x == 0 && threadIdx.x < 3) a.scalars[PAGE_TRACE_AT + PAGE_PHASES + 1 + threadIdx.x] = 0;
   if (want_fr) grid_zero16(a.fb.btable, a.bslots * 8);
   grid.sync();
@@ -77,20 +76,20 @@ __global__ void __launch_bounds__(CTA_THREADS, 2) yt_page_kernel(const __grid_co
   stamp();
 
   // P3
-  if (want_json && blockIdx.x == 0) cta_scan_u32(a.yo.linelen, n, a.line_off, a.scalars + a.sc_line_total);
-  if (want_links && blockIdx.x == 1 % gridDim.x) cta_scan_u32(a.yo.link_count, n, a.link_off, a.scalars + a.sc_link_total);
+  if (want_json && blockIdx.x == 0) cta_scan_u32(a.yo.linelen, n, a.line_off, a.scalars + SC_LINE_TOTAL);
+  if (want_links && blockIdx.x == 1 % gridDim.x) cta_scan_u32(a.yo.link_count, n, a.link_off, a.scalars + SC_LINK_TOTAL);
   if (want_fr) frontier_count_body(n, a.yo.link_start, a.yo.link_count, a.fb, t0, nt);
   grid.sync();
   stamp();
 
   // P4
   if (want_fr) {
-    if (blockIdx.x == last) cta_scan_u32(a.fb.rec_new, n, a.new_off, a.scalars + a.sc_new);
+    if (blockIdx.x == last) cta_scan_u32(a.fb.rec_new, n, a.new_off, a.scalars + SC_NEW);
     grid.sync();
   }
   stamp();
-  const uint64_t links_bytes = want_links ? (a.scalars[a.sc_link_total] * sizeof(tgi_link) + 255) & ~255ull : 0;
-  const uint64_t line_total = want_json ? a.scalars[a.sc_line_total] : 0;
+  const uint64_t links_bytes = want_links ? (a.scalars[SC_LINK_TOTAL] * sizeof(tgi_link) + 255) & ~255ull : 0;
+  const uint64_t line_total = want_json ? a.scalars[SC_LINE_TOTAL] : 0;
   if (links_bytes + line_total > a.var_cap || (a.max_out && line_total > a.max_out)) {
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(a.yo.err, ERR_PAGE_OVERFLOW);
     return;
@@ -110,7 +109,7 @@ __global__ void __launch_bounds__(CTA_THREADS, 2) yt_page_kernel(const __grid_co
 
   // P6
   if (want_links) links_compact_body(n, a.yo.link_start, a.yo.link_count, a.link_off, a.yo.arena, (tgi_link*)a.var, a.link_off32);
-  if (want_fr && blockIdx.x == last && threadIdx.x == 0) frontier_commit_body(a.fr, a.new_off, n, a.scalars + a.sc_new, a.yo.err);
+  if (want_fr && blockIdx.x == last && threadIdx.x == 0) frontier_commit_body(a.fr, a.new_off, n, a.scalars + SC_NEW, a.yo.err);
   stamp();
 }
 
